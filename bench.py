@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric (Falcon-40B Q4_K decode tokens/s on B200) and, beside it, every BASELINE config.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config headline|1|2|3|4|5] [--no-extras]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config headline|1|2|3|4|5] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (N > 1)
 
 A "step" is one decode eval (one token, n_batch = 1) of a synthetic random-init Falcon model through the hot path; weights are
@@ -373,8 +373,9 @@ class Ctx:
         return f
 
 
-def decode_leg(cx, f, hp, wtype, steps, warmup, pos0, rope, with_kernel_probe=True):
-    """-> dict of the decode figures of one model (see module docstring).  All ranks call it; figures are max-over-ranks times."""
+def decode_leg(cx, f, hp, wtype, steps, warmup, pos0, rope, with_kernel_probe=True, keep_output=False):
+    """-> dict of the decode figures of one model (see module docstring).  All ranks call it; figures are max-over-ranks times.
+    keep_output (one GPU): "_output" holds the logits the last timed step left on the device."""
     L, b = cx.L, cx.b
     stream = f.stream()
     tok_dev = b.DevBuf(src=np.array([1234], np.int32))
@@ -403,6 +404,10 @@ def decode_leg(cx, f, hp, wtype, steps, warmup, pos0, rope, with_kernel_probe=Tr
     wall_ms = (time.perf_counter() - t0) * 1e3
     tf_ms = L.b200_event_elapsed_ms(e0, e1)
     launches = f.last_launches() * steps
+    output = None
+    if keep_output:
+        output = np.empty(hp["n_vocab"], np.float32)
+        L.b200_memcpy_d2h(output.ctypes.data_as(C.c_void_p), f.logits_dev(), output.nbytes)
 
     # ---- (2) N > 1: strict autoregressive, device-side (arg-max on the last rank, id -> rank 0 over NCCL inside the step graph)
     auto_ms = None
@@ -451,6 +456,8 @@ def decode_leg(cx, f, hp, wtype, steps, warmup, pos0, rope, with_kernel_probe=Tr
         out["pipelined_tok_s"] = steps / (tf_ms / 1e3)
         out["autoregressive_tok_s"] = value
     out["_probe"] = probe
+    if keep_output:
+        out["_output"] = output
     return out
 
 
@@ -465,7 +472,7 @@ def prompt_leg(cx, f, hp, n_tokens=2048, n_batch=512):
     t0 = time.perf_counter()
     dev_ms = 0.0
     for c in range(n_tokens // n_batch):
-        f.eval(toks[n_batch * c: n_batch * (c + 1)], n_batch * c, 0)
+        logits = f.eval(toks[n_batch * c: n_batch * (c + 1)], n_batch * c, 0)
         dev_ms += f.last_ms()
     cx.barrier(stream)
     wall_s = time.perf_counter() - t0
@@ -483,11 +490,13 @@ def prompt_leg(cx, f, hp, n_tokens=2048, n_batch=512):
                          "what": "whole prompt (dequantising tcgen05 GEMMs + tcgen05 attention) per GPU against the sustained dense bf16 peak; "
                                  + ("device time (CUDA events per eval)" if cx.world == 1 else "wall clock (pipelined chunks)")},
             "roofline_tok_s": tf_peak * 1e12 * cx.world / ((mm_flop + att_flop) / n_tokens),
-            "what": "%d x b200_falcon_eval of %d host tokens; tok_s = wall clock incl. H2D / D2H" % (n_tokens // n_batch, n_batch)}
+            "what": "%d x b200_falcon_eval of %d host tokens; tok_s = wall clock incl. H2D / D2H" % (n_tokens // n_batch, n_batch),
+            "_output": logits[0]}
 
 
 def matvec_leg(cx, K=4096, M=4096, n_mats=32, reps=20, cpu=True):
-    """BASELINE config 1 on the GPU (+ the reference's ggml.c on the host cores): same blocks, same activation column"""
+    """BASELINE config 1 on the GPU (+ the reference's ggml.c on the host cores): same blocks, same activation column.
+    "_output" holds the result column of the last timed call."""
     L, b = cx.L, cx.b
     import ggllm_cpp_b200.ggcc as ggcc
     if cpu:
@@ -510,6 +519,7 @@ def matvec_leg(cx, K=4096, M=4096, n_mats=32, reps=20, cpu=True):
     L.b200_event_record(e1, None)
     L.b200_event_synchronize(e1)
     us = L.b200_event_elapsed_ms(e0, e1) * 1e3 / (reps * n_mats)
+    y_last = yd.download(np.float32, (M,))
     # end to end: host activation column in, host result out (H2D + quantise + mat-vec + D2H), what ggml_cuda_mul_mat's caller sees
     xh, yh = np.ascontiguousarray(x[None, :]), np.zeros((1, M), np.float32)
     t0 = time.perf_counter()
@@ -527,7 +537,7 @@ def matvec_leg(cx, K=4096, M=4096, n_mats=32, reps=20, cpu=True):
            "gpu": {"us_per_call": us, "GBs": nbytes / us / 1e3, "frac_of_hbm_peak": nbytes / us / 1e3 / peak, "GFLOPs": 2.0 * K * M / us / 1e3,
                    "e2e_us_per_call": e2e_us, "e2e_bytes": {"h2d": K * 4, "d2h": M * 4}, "roofline_us": nbytes / peak / 1e3,
                    "note": "a 9.4 MB mat-vec lasts ~2 us: back-to-back launches are launch-latency bound, not HBM bound"},
-           "cpu": ref}
+           "cpu": ref, "_output": y_last}
     if y_cpu is not None:
         mag = float(np.abs(y_cpu).max())
         out["parity_max_abs_diff_over_max"] = float(np.abs(y_gpu - y_cpu).max() / mag)
@@ -562,6 +572,14 @@ def pipeline_parity(cx):
             "checked": "16-token prompt (all logits) + 4 decode evals + 12 greedy tokens generated through the ring, last rank vs 1-rank engine"}
 
 
+def dump_outputs(out_dir, arrays):
+    """DIR/<name>.npy in float32, so that two builds run with the same arguments can be compared output for output (the inputs are
+    seeded); the arrays here are a few hundred KB at most"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -572,8 +590,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="only the selected config (skip the other BASELINE configs and the CPU baseline)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--layers", type=int, default=0, help="debug: fewer layers than the real model (the result is then NOT a valid bench value)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                                                          "(float32): the logits of a decode or prompt config, the result column of config 1")
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (world > 1 or args.impl != "b200"):
+        ap.error("--dump-outputs needs a single-GPU run of --impl b200")
     warmup = max(args.warmup, 3)
     sel = args.config
     dsel = sel if sel in DECODE_CONFIGS else "headline"
@@ -616,12 +638,15 @@ def main():
     out_extra = {}
 
     if sel == "1":
-        r = matvec_leg(cx, cpu=not args.no_cpu_baseline) if cx.rank == 0 else None
+        r = matvec_leg(cx, reps=args.steps, cpu=not args.no_cpu_baseline) if cx.rank == 0 else None
         if cx.rank == 0:
+            y = r.pop("_output")
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, {"y": y})
             print(json.dumps({"metric": "q4_0_4096x4096_matvec_us", "value": r["gpu"]["us_per_call"], "unit": "us", "n_gpus": args.gpus, "steps": args.steps, "warmup": warmup,
                               "ms_per_step": r["gpu"]["us_per_call"] / 1e3, "higher_is_better": False, "scaling": "weak", "vs_baseline": None, "dtype": "int8 x int4 block dots (dp4a)",
                               "data": "synthetic", "config": config, "e2e": {"value": r["gpu"]["e2e_us_per_call"], "unit": "us", "h2d_bytes_per_step": 4096 * 4, "d2h_bytes_per_step": 4096 * 4},
-                              "gpu_launches": 20 * 32, "roofline": {"bound": "hbm", "achieved": r["gpu"]["GBs"], "peak": peak, "unit": "GB/s", "frac": r["gpu"]["frac_of_hbm_peak"], "traffic": None},
+                              "gpu_launches": args.steps * r["n_mats"], "roofline": {"bound": "hbm", "achieved": r["gpu"]["GBs"], "peak": peak, "unit": "GB/s", "frac": r["gpu"]["frac_of_hbm_peak"], "traffic": None},
                               "cpu_baseline": {"value": r["cpu"]["us_per_call"], "unit": "us", "cores": r["cpu"]["cores"], "kind": r["cpu"]["kind"], "sample": "32 rotating matrices x 8 passes"} if r["cpu"] else None,
                               "detail": r}))
         return
@@ -629,12 +654,16 @@ def main():
     n_batch = 512 if (sel in ("headline", "3") and extras or sel == "3") else 1
     sampler = ClockSampler(cx.local_rank)
     f = cx.make_model(hp, wtype, n_ctx, n_batch)
-    d = decode_leg(cx, f, hp, wtype, args.steps, warmup, pos0, rope)
+    d = decode_leg(cx, f, hp, wtype, args.steps, warmup, pos0, rope, keep_output=bool(args.dump_outputs) and sel != "3")
     clocks = sampler.stop()
-    prompt = None
+    prompt, prompt_output = None, None
     if n_batch >= 512:
         prompt = prompt_leg(cx, f, hp)
+        prompt_output = prompt.pop("_output", None)
     f.free()
+    decode_output = d.pop("_output", None)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": prompt_output if sel == "3" else decode_output})
     parity = pipeline_parity(cx) if cx.world > 1 else None
 
     if extras and sel == "headline":
@@ -655,6 +684,7 @@ def main():
         if cx.rank == 0:
             try:
                 out_extra["cfg1"] = matvec_leg(cx, cpu=not args.no_cpu_baseline)
+                out_extra["cfg1"].pop("_output", None)
             except Exception as ex:
                 out_extra["cfg1"] = {"error": repr(ex)}
     if cx.rank != 0:

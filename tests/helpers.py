@@ -1,4 +1,5 @@
 """Shared test helpers: synthetic random-init Falcon models (SURVEY.md section 8d row 2) quantised by the oracle."""
+import hashlib
 import os
 import sys
 import numpy as np
@@ -38,6 +39,42 @@ def synth_model(hp, wtype, seed=1234, embed_type=None, overrides=None):
                     t = ot
             tensors[name] = (t, ne, w if t == po.F32 else w.astype(np.float16) if t == po.F16 else o.quantize(t, w))
     return tensors
+
+
+def digest(a):
+    """SHA-256 of an array's bytes: how tests/golden stores reference outputs that are compared bit for bit but too large to keep"""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+# the sampler-chain cases of tests/test_sampling_gpu.py: (top_k, top_p, temp, repeat_penalty, repeat_last_n)
+SAMPLER_CASES = [(40, 0.95, 0.8, 1.1, 64), (1, 1.0, 0.8, 1.0, 0), (200, 0.5, 1.3, 1.3, 16), (40, 1.0, 0.0, 1.2, 64), (7, 0.9, 0.7, 1.0, 0),
+                 (1000, 0.999, 2.0, 1.05, 200)]
+
+
+def codec_random_inputs(t):
+    """-> [(scale, x)]: the random rows the codecs of type t are checked on, 8 x 2048 N(0, scale^2) per scale, the first 300 values of
+    row 0 zero"""
+    rng = np.random.default_rng(t)
+    out = []
+    for scale in (1.0, 0.02, 30.0):
+        x = (rng.standard_normal((8, 2048)) * scale).astype(np.float32)
+        x[0, :300] = 0
+        out.append((scale, x))
+    return out
+
+
+def sampler_case(top_k, last_n, n_vocab=65024):
+    """the seeded inputs of one sampler-chain case: (100-id history, next_logits(window) -> the next float32 logits row)"""
+    rng = np.random.default_rng(top_k + last_n)
+    history = [int(v) for v in rng.integers(0, n_vocab, size=100)]
+
+    def next_logits(window):
+        logits = (rng.standard_normal(n_vocab) * 3.0).astype(np.float32)
+        logits[rng.integers(0, n_vocab, size=5)] += 6.0                      # a few dominant candidates, like real logits
+        if window:
+            logits[window[-1]] += 5.0                                       # make the penalty matter: the last id stays attractive
+        return logits
+    return history, next_logits
 
 
 def write_synth(path, hp, wtype, seed=1234):

@@ -1,6 +1,6 @@
 import sys, os
 import numpy as np
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import ggllm_cpp_b200.binding as b
 b.init(0); L = b.lib()
 K, M, mode = int(sys.argv[1]), int(sys.argv[2]), int(sys.argv[3])
